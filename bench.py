@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- train-step throughput (frames/s) of the colvars-finder step on B200, one JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c1|c4] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c1|c4] [--impl reference] [--dump-outputs DIR]
 
 A step is the body of the reference's mini-batch loop (core.py:498-522 / 699-712): zero_grad, loss,
 backward, optimizer.step -- through the drop-in classes, on one batch of synthetic frames per GPU
@@ -23,21 +23,31 @@ Weak scaling: every rank keeps `--frames` frames (default 2^22, 1.1 GB > L2) res
 `cpu_baseline` / `--impl reference`: oracle/ref_torch.py (restatement of the reference's PyTorch path; /root/reference does
             not exist on the GPU box) on the host cores, on a bounded sample of the same workload.  Only these two legs
             import oracle/.
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the last timed step computed to DIR/<name>.npy (float32 or
+            float64): the step's return values, every parameter gradient and every parameter after the optimizer update
+            (see dump_outputs).  The inputs depend on the arguments only, so two builds can be compared output for output.
+
+The library must have been built (__graft_entry__.build()) from the sources next to it; bench.py compiles nothing and writes
+nothing into the tree (the tasks' log directory is a temporary directory).
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import gc
 import signal
 import ctypes as C
 import json
 import os
+import shutil
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
+sys.dont_write_bytecode = True      # the tree may be read-only and is left as build() made it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "colvars-finder_b200")):
     if p not in sys.path:
@@ -206,12 +216,15 @@ def measured_peaks():
 
 
 def build_workload(name, n_frames, dev, seed, lr=1e-3):
-    """Returns (step_fn(X, w) -> loss tensor, X, w, task)."""
+    """Returns (step_fn(X, w) -> loss tensor, X, w, task).  step_fn.last holds what the caller of the step's path received in
+    the latest call (the return values of loss_func / weighted_MSE_loss / Align), by name."""
     from colvarsfinder import core, nn, utils
     import bench_data as bd
     FakeTrajectory = bd.SyntheticTrajectory
     torch.manual_seed(2026)
-    tmp = f"/tmp/cvf_bench_{os.getpid()}"
+    tmp = tempfile.mkdtemp(prefix="cvf_bench_")
+    atexit.register(shutil.rmtree, tmp, ignore_errors=True)
+    last = {}
     if name == "c2p":
         base = bd.DIPEPTIDE_NM * 10.0
         X = bd.frames(base, n_frames, dev, seed)
@@ -221,7 +234,9 @@ def build_workload(name, n_frames, dev, seed, lr=1e-3):
         out = torch.empty_like(X)
 
         def step(Xb, wb):
-            return align(Xb, out=out)[0, 0, 0]
+            last["aligned"] = align(Xb, out=out)
+            return last["aligned"][0, 0, 0]
+        step.last = last
         return step, X, w, None
     if name in ("c3", "c2"):
         base = bd.DIPEPTIDE_NM * 10.0
@@ -268,18 +283,51 @@ def build_workload(name, n_frames, dev, seed, lr=1e-3):
     if isinstance(task, core.EigenFunctionTask):
         def step(Xb, wb):
             task.optimizer.zero_grad(set_to_none=True)
-            loss = task.loss_func(Xb, wb, None, None)[0]
-            loss.backward()
+            out = task.loss_func(Xb, wb, None, None)
+            out[0].backward()
             task.optimizer.step()
-            return loss
+            last["loss"], last["eig"], last["obj"], last["pen"], last["cvec"] = out
+            return out[0]
     else:
         def step(Xb, wb):
             task.optimizer.zero_grad(set_to_none=True)
             loss = task.weighted_MSE_loss(Xb, wb)
             loss.backward()
             task.optimizer.step()
+            last["loss"] = loss
             return loss
+    step.last = last
     return step, X, w, task
+
+
+DUMP_MAX_ELEMENTS = 1 << 22     # per array; larger outputs are sampled by rows
+DUMP_MAX_BYTES = 64 << 20       # all files together
+
+
+def dump_outputs(path, step, task):
+    """Write what the latest call of `step` computed to path/<name>.npy: the tensors in step.last, then grad.<parameter>
+    and param.<parameter> (the gradient of that step and the parameter after its optimizer update) for every parameter of
+    the model.  float64 stays float64, everything else is written as float32.  An array of more than DUMP_MAX_ELEMENTS
+    elements is replaced by the rows np.random.default_rng(0).choice(rows, m, replace=False), sorted, with m the largest row
+    count that fits: the same rows for the same shape in every run."""
+    arrays = dict(step.last)
+    if task is not None:
+        for name, p in task.model.named_parameters():
+            if p.grad is not None:
+                arrays[f"grad.{name}"] = p.grad
+            arrays[f"param.{name}"] = p
+    os.makedirs(path, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        if a.size > DUMP_MAX_ELEMENTS:
+            m = max(1, DUMP_MAX_ELEMENTS // (a.size // a.shape[0]))
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], m, replace=False))]
+        total += a.nbytes
+        if total > DUMP_MAX_BYTES:
+            raise SystemExit(f"--dump-outputs: the outputs exceed {DUMP_MAX_BYTES >> 20} MB at {name}")
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------ CPU arm
@@ -441,7 +489,11 @@ def main():
     ap.add_argument("--cpu-frames", type=int, default=None, help="frames per step of the CPU sample (default 100000; 4096 for c5)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--strong", action="store_true", help="also time the 2^23-frame global batch of SURVEY 8d at N = 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, world, local = dist_env()
     if args.frames is None:
         args.frames = 1 << 16 if args.workload == "c5" else 1 << 22
@@ -474,15 +526,14 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device (the product path has no CPU fallback)")
     import __graft_entry__ as entry
-    if rank == 0:
-        entry.build()
+    if entry.library_hash() != entry.source_hash():
+        raise SystemExit(f"{entry.LIB} is missing or was built from other sources: run __graft_entry__.build() first")
     dev = torch.device("cuda", local)
     torch.cuda.set_device(dev)
     if world > 1:
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=dev)
         dist.barrier()
-    entry.build()
     from colvarsfinder import _lib
 
     # started early: nvidia-smi takes a while to deliver its first row (CVF_BENCH_CLOCKS=0 switches the sampling off)
@@ -530,6 +581,8 @@ def main():
     value = args.frames * world * K / (ms_total * 1e-3)
     final_loss = float(loss.detach())
     launches_timed = sum(v[2] for v in _lib.profile_read(reset=True).values())
+    if args.dump_outputs and rank == 0:      # before the steps below change the parameters
+        dump_outputs(args.dump_outputs, step, task)
 
     # ---- end to end: batch in pinned host memory, H2D + step + D2H(loss) per step, copy of step i+1 overlapped
     numa = bind_to_gpu_numa_node(local) if world > 1 else "single process: not bound"

@@ -1,5 +1,6 @@
-import sys, time, torch
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/colvars-finder_b200')
+import os, sys, time, torch
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'colvars-finder_b200'))
 import __graft_entry__ as g; g.build()
 import bench, gc
 dev = torch.device('cuda', 0)
