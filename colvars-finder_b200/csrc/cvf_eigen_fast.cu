@@ -1600,7 +1600,9 @@ pass2_kernel(const FastPlan P, const float* __restrict__ w, const double* __rest
   // deterministic), into an fp64 vector in the shared memory the operand rows no longer need; networks whose totals went to
   // per-warp vectors in global memory by atomics (beyond tm_nets) are folded in after them; one vector per CTA leaves the SM
   __syncthreads();
-  double* acc = reinterpret_cast<double*>(rows0);   // [tm_nets * n_params]: at most three networks' parameters, far below the rows' size
+  // [tm_nets * n_params]: up to kMaxK networks keep totals in tensor memory (e.g. [12,20,20,1] with k = 8); for every shape the
+  // host accepts, their vectors take at most 43% of the operand rows (worst case [48,20,20,20,1], k = 7: 4 networks, 6 warps)
+  double* acc = reinterpret_cast<double*>(rows0);
   const int n_acc = tm_nets * P.n_params;
   for (int i = tid; i < n_acc; i += nt) acc[i] = 0.0;
   __syncthreads();
@@ -1959,7 +1961,9 @@ static int run_grad(const cvf_preproc* pp, const NetPlan& np, int k, const float
   }
   const size_t smem2 = pass2_smem_bytes(k, P.img2_floats, P.geo_floats, P.d_rp, H, NH, nw);
   if ((size_t)3 * np.n_params * sizeof(double) > (size_t)nw * pass2_rows_per_warp(P.d_rp, H, NH) * kRowPad * sizeof(float)) {
-    set_error("fast eigen path: the operand rows cannot hold the CTA's gradient vector");   // 3 networks at most keep totals in TMEM
+    // a floor, not the exact fold size: up to kMaxK networks keep totals in TMEM, and the fold of pass2_kernel fits the rows of
+    // every supported shape (its comment)
+    set_error("fast eigen path: the operand rows cannot hold the CTA's gradient vector");
     return CVF_E_UNSUPPORTED;
   }
   const long long n_tiles = P.Bp / 32;
