@@ -41,6 +41,8 @@ SYMBOLS = {
     "cvf_mlp_param_count": (_I64, [C.POINTER(Mlp)]),
     "cvf_align_fwd": (C.c_int, [_P, _I64, _I32, _P, _I32, _P, _P, _P, _P, _P]),
     "cvf_features_fwd": (C.c_int, [_P, _I64, C.POINTER(Preproc), _P, _P]),
+    "cvf_align_vjp": (C.c_int, [_P, _I64, _I32, _P, _I32, _P, _P, _P, _P]),
+    "cvf_features_vjp": (C.c_int, [_P, _I64, C.POINTER(Preproc), _P, _P, _P]),
     "cvf_eigen_num_stats": (_I32, [_I32]),
     "cvf_eigen_num_combine": (_I32, [_I32]),
     "cvf_eigen_workspace_bytes": (_SZ, [C.POINTER(Preproc), C.POINTER(Mlp), _I32, _I64]),

@@ -9,7 +9,13 @@ Operators (each with ``register_fake`` for shape inference and ``register_autogr
 * ``cvf::eigen_loss(X, w, params, handle) -> (y, comb)``           the two above fused (EigenFunctionTask's generator loss)
 * ``cvf::eigen_tlag_sx``, ``cvf::eigen_tlag_combine``              transfer-operator branch (core.py:412-416,428,440)
 * ``cvf::ae_sums(F, T, w, params, want_grad, handle) -> (sums, gsum)``  weighted reconstruction error and its gradient
-* ``cvf::align_fwd(x, ref, idx) -> y``                             Kabsch alignment (stand-alone pre-pass)
+* ``cvf::align_fwd(x, ref, idx) -> y``                             Kabsch alignment (stand-alone pre-pass); backward =
+  ``cvf::align_vjp(x, ref, idx, g_y) -> g_x``
+* ``cvf::features_fwd(x, handle) -> r``                            features (after alignment) of a PreprocSpec; backward =
+  ``cvf::features_vjp(x, g_r, handle) -> g_x``
+
+The two ``*_vjp`` operators are first-order only: they have no autograd formula, so differentiating a gradient that passed
+through them raises instead of returning a zero or partial second derivative.
 
 ``handle`` is an integer naming the host-side context (descriptors + scratch) of a task: operators take tensors and plain
 scalars only.
@@ -174,6 +180,7 @@ class PreprocSpec:
                 s.diag = self._dev(g)
             self.d_r = d_r
         self.struct = s
+        self.handle = _register_context(self)      # the ``handle`` of cvf::features_fwd / cvf::features_vjp
 
     def _dev(self, t):
         t = t.contiguous().to(self.device)
@@ -756,8 +763,19 @@ def ae_loss(actx: AEContext, F, weight, target=None):
 
 
 # ------------------------------------------------------------------------------------------ alignment
+def check_align_args(x, ref, align_idx, what):
+    """The kernels dereference ref and align_idx on the device of x: a module left on the host (Align(...) without .to(device))
+    is refused here instead of faulting on the GPU."""
+    if ref.device != x.device or align_idx.device != x.device:
+        raise RuntimeError(f"{what}: the reference and alignment indices live on {ref.device} / {align_idx.device}, the frames "
+                           f"on {x.device}: move the module to the frames' device (.to(device))")
+    if ref.dtype != torch.float32 or align_idx.dtype != torch.int32 or ref.numel() != 3 * align_idx.numel():
+        raise RuntimeError(f"{what}: reference must be float32 [n_align,3] and alignment indices int32 [n_align]")
+
+
 @torch.library.custom_op("cvf::align_fwd", mutates_args=())
 def align_fwd_op(x: torch.Tensor, ref: torch.Tensor, align_idx: torch.Tensor) -> torch.Tensor:
+    check_align_args(x, ref, align_idx, "cvf::align_fwd")
     y = torch.empty_like(x)
     with torch.cuda.device(x.device):
         _lib.check(_lib.lib().cvf_align_fwd(x.data_ptr(), x.shape[0], x.shape[1], align_idx.data_ptr(), align_idx.numel(),
@@ -768,3 +786,87 @@ def align_fwd_op(x: torch.Tensor, ref: torch.Tensor, align_idx: torch.Tensor) ->
 @align_fwd_op.register_fake
 def _(x, ref, align_idx):
     return torch.empty_like(x)
+
+
+@torch.library.custom_op("cvf::align_vjp", mutates_args=())
+def align_vjp_op(x: torch.Tensor, ref: torch.Tensor, align_idx: torch.Tensor, g_y: torch.Tensor) -> torch.Tensor:
+    """(dy/dx)^T g_y of cvf::align_fwd.  No autograd formula of its own: differentiating it again raises."""
+    check_align_args(x, ref, align_idx, "cvf::align_vjp")
+    if g_y.shape != x.shape or g_y.dtype != torch.float32 or not g_y.is_contiguous() or g_y.device != x.device:
+        raise RuntimeError("cvf::align_vjp: g_y must be a contiguous float32 tensor of the frames' shape and device")
+    g_x = torch.empty_like(x)
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib().cvf_align_vjp(x.data_ptr(), x.shape[0], x.shape[1], align_idx.data_ptr(), align_idx.numel(),
+                                            ref.data_ptr(), g_y.data_ptr(), g_x.data_ptr(), _stream()), "cvf_align_vjp")
+    return g_x
+
+
+@align_vjp_op.register_fake
+def _(x, ref, align_idx, g_y):
+    return torch.empty_like(x)
+
+
+def _align_fwd_setup(ctx, inputs, output):
+    x, ref, align_idx = inputs
+    ctx.save_for_backward(x, ref, align_idx)
+
+
+def _align_fwd_backward(ctx, g_y):
+    x, ref, align_idx = ctx.saved_tensors
+    # the cotangent of .sum() and friends is an expanded view (stride 0): the kernel reads dense frames
+    return align_vjp_op(x, ref, align_idx, g_y.contiguous()), None, None
+
+
+align_fwd_op.register_autograd(_align_fwd_backward, setup_context=_align_fwd_setup)
+
+
+# ------------------------------------------------------------------------------------------ features
+# ``handle`` names a PreprocSpec (PreprocSpec.handle).  utils.FeatureMap builds a temporary Preprocessing, and
+# with it a temporary spec, on every call: the autograd context keeps the spec alive until backward has run, and backward uses
+# that same spec -- alignment_elided included -- so it differentiates the function the forward computed.
+@torch.library.custom_op("cvf::features_fwd", mutates_args=())
+def features_fwd_op(x: torch.Tensor, handle: int) -> torch.Tensor:
+    spec = _context(handle)
+    r = torch.empty(x.shape[0], spec.d_r, device=x.device, dtype=torch.float32)
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib().cvf_features_fwd(x.data_ptr(), x.shape[0], spec.struct_ptr(), r.data_ptr(), _stream()),
+                   "cvf_features_fwd")
+    return r
+
+
+@features_fwd_op.register_fake
+def _(x, handle):
+    return x.new_empty((x.shape[0], _context(handle).d_r))
+
+
+@torch.library.custom_op("cvf::features_vjp", mutates_args=())
+def features_vjp_op(x: torch.Tensor, g_r: torch.Tensor, handle: int) -> torch.Tensor:
+    """(dr/dx)^T g_r of cvf::features_fwd.  No autograd formula of its own: differentiating it again raises."""
+    spec = _context(handle)
+    if tuple(g_r.shape) != (x.shape[0], spec.d_r) or g_r.dtype != torch.float32 or not g_r.is_contiguous() or g_r.device != x.device:
+        raise RuntimeError(f"cvf::features_vjp: g_r must be a contiguous float32 [{x.shape[0]},{spec.d_r}] tensor on the frames' device")
+    g_x = torch.empty_like(x)
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib().cvf_features_vjp(x.data_ptr(), x.shape[0], spec.struct_ptr(), g_r.data_ptr(), g_x.data_ptr(),
+                                               _stream()), "cvf_features_vjp")
+    return g_x
+
+
+@features_vjp_op.register_fake
+def _(x, g_r, handle):
+    return torch.empty_like(x)
+
+
+def _features_fwd_setup(ctx, inputs, output):
+    x, handle = inputs
+    ctx.save_for_backward(x)
+    ctx.handle = handle
+    ctx.spec = _context(handle)      # strong reference: the registry only holds weak ones
+
+
+def _features_fwd_backward(ctx, g_r):
+    x, = ctx.saved_tensors
+    return features_vjp_op(x, g_r.contiguous(), ctx.handle), None
+
+
+features_fwd_op.register_autograd(_features_fwd_backward, setup_context=_features_fwd_setup)

@@ -7,8 +7,9 @@
   the third-party ``molann`` package (examples/dipeptide/main.ipynb:335-348).  Here they are descriptors:
   the task classes lower them into ``cvf_preproc`` and the CUDA kernels evaluate alignment, features and
   their (transpose-)Jacobians; calling the modules directly runs the stand-alone CUDA pre-pass
-  (``cvf_align_fwd`` / ``cvf_features_fwd``).  The integrators / weight calculators of the reference's
-  utils.py (data generation) are outside this package's scope.
+  (``cvf_align_fwd`` / ``cvf_features_fwd``), whose autograd backward is ``cvf_align_vjp`` / ``cvf_features_vjp`` (first
+  order: ``torch.autograd.grad(cv(x).sum(), x)`` works through ``colvar_model()``).  The integrators / weight calculators of
+  the reference's utils.py (data generation) are outside this package's scope.
 """
 from __future__ import annotations
 
@@ -122,6 +123,12 @@ def _stream_ptr():
     return torch.cuda.current_stream().cuda_stream
 
 
+def _recording(x):
+    """True when autograd records the call: grad mode is on and the input requires grad.  Only then do the layers go through
+    the cvf:: operators that carry the backward; otherwise they make the plain library call."""
+    return torch.is_grad_enabled() and x.requires_grad
+
+
 def _require_cuda_f32(x, what):
     if not (isinstance(x, torch.Tensor) and x.is_cuda):
         raise RuntimeError(f"{what}: input must be a CUDA tensor (this build has no CPU path)")
@@ -161,16 +168,18 @@ class Align(torch.nn.Module):
         print('\npositions of reference state used in aligment:\n', self.ref_pos.cpu().numpy())
 
     def forward(self, x, out=None):
-        """Aligned frames; ``out`` (optional, [B,N,3] float32 on the same device) receives them without an allocation."""
+        """Aligned frames; ``out`` (optional, [B,N,3] float32 on the same device) receives them without an allocation.
+        Differentiable in ``x`` (first order) when called without ``out``."""
         x = _require_cuda_f32(x, "Align")
         if x.dim() != 3 or x.shape[2] != 3:
             raise RuntimeError(f"Align expects [B,N,3], got {tuple(x.shape)}")
         if out is not None and (out.shape != x.shape or out.dtype != torch.float32 or out.device != x.device or not out.is_contiguous()):
             raise RuntimeError("Align: out must be a contiguous float32 tensor of the input's shape on the input's device")
-        if out is None:
-            from . import _ops      # registers the cvf:: operators
+        from . import _ops      # registers the cvf:: operators and their autograd formulas
+        _ops.check_align_args(x, self.ref_pos, self.align_idx, "Align")
+        if out is None and _recording(x):
             return torch.ops.cvf.align_fwd(x, self.ref_pos, self.align_idx)
-        y = out
+        y = torch.empty_like(x) if out is None else out
         with torch.cuda.device(x.device):
             _lib.check(_lib.lib().cvf_align_fwd(x.data_ptr(), x.shape[0], x.shape[1], self.align_idx.data_ptr(),
                                                 self.align_idx.numel(), self.ref_pos.data_ptr(), y.data_ptr(), None,
@@ -179,7 +188,9 @@ class Align(torch.nn.Module):
 
     def rotation(self, x):
         """Aligned frames plus the rotation R [B,3,3] and centroid c [B,3] of every frame."""
+        from . import _ops
         x = _require_cuda_f32(x, "Align")
+        _ops.check_align_args(x, self.ref_pos, self.align_idx, "Align.rotation")
         y = torch.empty_like(x)
         R = torch.empty(x.shape[0], 3, 3, device=x.device, dtype=torch.float32)
         c = torch.empty(x.shape[0], 3, device=x.device, dtype=torch.float32)
@@ -257,6 +268,8 @@ class Preprocessing(torch.nn.Module):
         if key not in self._spec_cache:
             self._spec_cache[key] = _ops.PreprocSpec(self, x.shape[1:], x.device, None)
         spec = self._spec_cache[key]
+        if _recording(x):
+            return torch.ops.cvf.features_fwd(x, spec.handle)
         out = torch.empty(x.shape[0], spec.d_r, device=x.device, dtype=torch.float32)
         with torch.cuda.device(x.device):
             _lib.check(_lib.lib().cvf_features_fwd(x.data_ptr(), x.shape[0], spec.struct_ptr(), out.data_ptr(),

@@ -40,7 +40,8 @@ static int device_attr(int* cache, cudaDeviceAttr attr, int fallback) {
 // ---- launch accounting -------------------------------------------------------------------------------------
 static const char* const g_kernel_names[K_COUNT] = {
     "align_fwd", "features_fwd", "eigen_stats(general)", "eigen_grad(general)", "eigen_combine", "reduce_partials", "ae_step",
-    "fast_pack", "fast_prep", "fast_pass1", "fast_stats", "fast_pass2", "(unused)", "fma_probe", "fast_jjt", "ae_fast_prep", "ae_fast_main", "ae_fast_dw", "weights_filter"};
+    "fast_pack", "fast_prep", "fast_pass1", "fast_stats", "fast_pass2", "(unused)", "fma_probe", "fast_jjt", "ae_fast_prep", "ae_fast_main", "ae_fast_dw", "weights_filter",
+    "align_vjp", "features_vjp"};
 static std::atomic<long long> g_launches[K_COUNT];
 static std::atomic<int> g_prof_on{0};
 static std::mutex g_prof_mutex;   // guards g_recs / g_n_recs (timed launches are a profiling mode, not the hot path)

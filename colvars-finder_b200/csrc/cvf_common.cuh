@@ -38,7 +38,7 @@ int max_smem_optin();
 enum KernelId {
   K_ALIGN = 0, K_FEATURES, K_EIGEN_STATS, K_EIGEN_GRAD, K_EIGEN_COMBINE, K_REDUCE, K_AE_STEP, K_FAST_PACK, K_FAST_PREP,
   K_FAST_PASS1, K_FAST_STATS, K_FAST_PASS2A, K_FAST_PASS2B, K_FMA_PROBE, K_FAST_JJT, K_AE_FAST_PREP, K_AE_FAST_MAIN, K_AE_FAST_DW,
-  K_WEIGHTS, K_COUNT
+  K_WEIGHTS, K_ALIGN_VJP, K_FEATURES_VJP, K_COUNT
 };
 void prof_begin(int id, cudaStream_t stream);
 void prof_end(int id, cudaStream_t stream);

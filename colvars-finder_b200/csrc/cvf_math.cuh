@@ -349,6 +349,77 @@ CVF_HD void cvf_dihedral(cvf_v3 p0, cvf_v3 p1, cvf_v3 p2, cvf_v3 p3, float& cs, 
   g[1] = (-1.0f - p) * g[0] + q * g[3];
   g[2] = p * g[0] + (-1.0f - q) * g[3];
 }
+// ---- adjoints (vector-Jacobian products) of one frame -----------------------------------------------------
+// Coordinate c of atom a of a frame sits at p[(3 a + c) * st]: st = 1 for a frame stored contiguously, the tile width for a
+// frame held as a column of a frame-minor tile.
+
+// Kabsch alignment y = (x - c) R (SURVEY 7.3-A, DESIGN §3): g holds G = dg/dy of the n atoms on entry and dg/dx on return,
+//   tau = sum_j G_j x y_j,  q = K^-1 tau,  dg/dx_j = (G_j - 1_A(j) (sum_j G_j / n_A + ref_j x q)) R^T
+// with A the alignment atoms aidx[0..n_align) (indices into the n atoms), ref their centred reference positions, R and K^-1
+// what cvf_rotation returns for the frame.  No SVD derivative: the rotation's response to x is the K^-1 solve.
+CVF_HD void cvf_align_vjp_frame(const float* y, float* g, int n, int st, const int* aidx, int n_align, const float* ref,
+                                const float* R, const float* Kinv) {
+  double t0 = 0, t1 = 0, t2 = 0, s0 = 0, s1 = 0, s2 = 0;
+  for (int a = 0; a < n; ++a) {
+    const float* p = y + 3 * a * st;
+    const float* q = g + 3 * a * st;
+    const double yx = p[0], yy = p[st], yz = p[2 * st], gx = q[0], gy = q[st], gz = q[2 * st];
+    t0 += gy * yz - gz * yy, t1 += gz * yx - gx * yz, t2 += gx * yy - gy * yx;
+    s0 += gx, s1 += gy, s2 += gz;
+  }
+  const cvf_v3 q = mul_sym(Kinv, v3((float)t0, (float)t1, (float)t2));
+  const double inv = 1.0 / n_align;
+  const cvf_v3 s = v3((float)(s0 * inv), (float)(s1 * inv), (float)(s2 * inv));
+  for (int a = 0; a < n_align; ++a) {
+    float* p = g + 3 * aidx[a] * st;
+    const cvf_v3 d = s + cross(v3(ref[3 * a], ref[3 * a + 1], ref[3 * a + 2]), q);
+    p[0] -= d.x, p[st] -= d.y, p[2 * st] -= d.z;
+  }
+  for (int a = 0; a < n; ++a) {
+    float* p = g + 3 * a * st;
+    const cvf_v3 o = mul_rowvec_T(v3(p[0], p[st], p[2 * st]), R);
+    p[0] = o.x, p[st] = o.y, p[2 * st] = o.z;
+  }
+}
+
+// Feature records (include/cvf.h: type, then up to 4 atom positions) evaluated on y: G += (dr/dy)^T u.  u[j * ust] is the
+// cotangent of output column j; G must hold zeros (or earlier contributions) on entry.  The stencils are the forward's.
+CVF_HD void cvf_features_vjp_frame(const float* y, float* G, int st, const int* feat, int n_feat, const float* u, int ust) {
+  auto ld = [&](int a) { return v3(y[3 * a * st], y[(3 * a + 1) * st], y[(3 * a + 2) * st]); };
+  auto add = [&](int a, cvf_v3 v) {
+    float* p = G + 3 * a * st;
+    p[0] += v.x, p[st] += v.y, p[2 * st] += v.z;
+  };
+  int col = 0;
+  for (int j = 0; j < n_feat; ++j) {
+    const int* fr = feat + 5 * j;
+    const int type = fr[0];
+    if (type == 0) {   // CVF_FEAT_POSITION
+      add(fr[1], v3(u[col * ust], u[(col + 1) * ust], u[(col + 2) * ust]));
+      col += 3;
+    } else if (type == 1) {   // CVF_FEAT_BOND
+      cvf_v3 gb;
+      cvf_bond(ld(fr[1]), ld(fr[2]), gb);
+      const cvf_v3 v = u[col * ust] * gb;
+      add(fr[2], v), add(fr[1], -1.0f * v);
+      col += 1;
+    } else if (type == 2) {   // CVF_FEAT_ANGLE
+      cvf_v3 ga, gc;
+      cvf_angle(ld(fr[1]), ld(fr[2]), ld(fr[3]), ga, gc);
+      const float w = u[col * ust];
+      add(fr[1], w * ga), add(fr[3], w * gc), add(fr[2], -w * (ga + gc));
+      col += 1;
+    } else {   // CVF_FEAT_DIHEDRAL: d cos = -sin dphi, d sin = cos dphi
+      float cs, sn;
+      cvf_v3 gp[4];
+      cvf_dihedral(ld(fr[1]), ld(fr[2]), ld(fr[3]), ld(fr[4]), cs, sn, gp);
+      const float w = cs * u[(col + 1) * ust] - sn * u[col * ust];
+      add(fr[1], w * gp[0]), add(fr[2], w * gp[1]), add(fr[3], w * gp[2]), add(fr[4], w * gp[3]);
+      col += 2;
+    }
+  }
+}
+
 // the same with the two middle gradients left implicit: g[1] = (-1-p) g0 + q g3, g[2] = p g0 + (-1-q) g3
 CVF_HD void cvf_dihedral_compact(cvf_v3 p0, cvf_v3 p1, cvf_v3 p2, cvf_v3 p3, float& cs, float& sn, cvf_v3& g0, cvf_v3& g3, float& p,
                                  float& q) {

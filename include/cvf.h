@@ -111,6 +111,16 @@ int cvf_align_fwd(const float* x, int64_t B, int32_t n_atoms, const int32_t* ali
 /* Whole-trajectory pre-pass of AutoEncoderTask.__init__ (core.py:635): r_out[B,d_r] = pp(x). */
 int cvf_features_fwd(const float* x, int64_t B, const cvf_preproc* pp, float* r_out, void* stream);
 
+/* Vector-Jacobian products of the two calls above: the autograd backward of utils.Align / FeatureMap / Preprocessing, which
+ * replaces the backward of molann's alignment and feature layers that torch.autograd.grad(y, X) runs at core.py:424.
+ * First order only.  The rotation is recomputed from x (the forward keeps nothing).
+ * cvf_align_vjp:    g_y [B,n_atoms,3] = dg/dy  ->  g_x [B,n_atoms,3] = dg/dx; same arguments and checks as cvf_align_fwd.
+ * cvf_features_vjp: g_r [B,d_r] = dg/dr  ->  g_x [B,n_atoms,3] = dg/dx for a kind-1 descriptor, with or without alignment;
+ *                   atoms that no record reads get exact zeros. */
+int cvf_align_vjp(const float* x, int64_t B, int32_t n_atoms, const int32_t* align_idx, int32_t n_align,
+                  const float* ref_centred, const float* g_y, float* g_x, void* stream);
+int cvf_features_vjp(const float* x, int64_t B, const cvf_preproc* pp, const float* g_r, float* g_x, void* stream);
+
 /* ---- EigenFunctionTask.loss_func, generator branch (core.py:387-457) split at its batch sums ---- */
 
 /* doubles in the stats vector: S0, S1[k], S2[k*k], SD[k] */
