@@ -73,6 +73,24 @@ def rel_l2(a, b):
     return float(np.linalg.norm(a - b) / n) if n > 0 else float(np.linalg.norm(a - b))
 
 
+def repeated_batch(D, B, seed, offset=0, device=None):
+    """(X, w, w_agg, idx): X = D[idx] on the device with idx uniform over the M frames of D, random fp32 weights w, and the
+    fp64 weight each distinct frame carries in total (host).  offset=1 returns a contiguous view that starts one frame into
+    its allocation (not 16-byte aligned for 12 N-byte frames with N = 2 mod 4)."""
+    import torch
+    device = torch.device("cuda", 0) if device is None else device
+    D = torch.as_tensor(D, device=device)
+    g = torch.Generator(device=device).manual_seed(seed)
+    idx = torch.randint(0, D.shape[0], (B,), generator=g, device=device)
+    w = torch.exp(0.5 * torch.randn(B, generator=g, device=device)).contiguous()
+    buf = torch.empty((B + offset,) + tuple(D.shape[1:]), dtype=D.dtype, device=device)
+    X = buf[offset:]
+    torch.index_select(D, 0, idx, out=X)
+    assert X.is_contiguous() and X.data_ptr() == buf.data_ptr() + offset * X[0].numel() * X.element_size()
+    w_agg = torch.zeros(D.shape[0], dtype=torch.float64, device=device).index_add_(0, idx, w.double())
+    return X, w, w_agg.cpu().numpy(), idx
+
+
 def tol(gold, ref32, rel=1e-5, slack=1.0):
     """SURVEY 7.3-D: pass when |ours-gold| <= max(rel*|gold|, slack*|ref32-gold|)."""
     return max(rel * abs(float(gold)), slack * abs(float(ref32) - float(gold)))

@@ -50,20 +50,7 @@ def release_memory():
 
 
 # --------------------------------------------------------------------------------------------- helpers
-def repeated_batch(D, B, seed, offset=0):
-    """(X, w, w_agg, idx): X = D[idx] on the device with idx uniform over the M frames of D, random fp32 weights w, and the
-    fp64 weight each distinct frame carries in total (host).  offset=1 returns a contiguous view that starts one frame into
-    its allocation (not 16-byte aligned for 12 N-byte frames with N = 2 mod 4)."""
-    D = torch.as_tensor(D, device=DEV)
-    g = torch.Generator(device=DEV).manual_seed(seed)
-    idx = torch.randint(0, D.shape[0], (B,), generator=g, device=DEV)
-    w = torch.exp(0.5 * torch.randn(B, generator=g, device=DEV)).contiguous()
-    buf = torch.empty((B + offset,) + tuple(D.shape[1:]), dtype=D.dtype, device=DEV)
-    X = buf[offset:]
-    torch.index_select(D, 0, idx, out=X)
-    assert X.is_contiguous() and X.data_ptr() == buf.data_ptr() + offset * X[0].numel() * X.element_size()
-    w_agg = torch.zeros(D.shape[0], dtype=torch.float64, device=DEV).index_add_(0, idx, w.double())
-    return X, w, w_agg.cpu().numpy(), idx
+repeated_batch = C.repeated_batch
 
 
 def schedule(B, k):
