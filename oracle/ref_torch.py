@@ -59,9 +59,9 @@ def mlp(params: Sequence[torch.Tensor], x: torch.Tensor, act=torch.tanh) -> torc
     return h
 
 
-def eigen_forward(nets: Sequence[Sequence[torch.Tensor]], r: torch.Tensor) -> torch.Tensor:
+def eigen_forward(nets: Sequence[Sequence[torch.Tensor]], r: torch.Tensor, act=torch.tanh) -> torch.Tensor:
     """k scalar nets evaluated on the same features and concatenated -> [B, k] (nn.py:293)."""
-    return torch.cat([mlp(p, r) for p in nets], dim=1)
+    return torch.cat([mlp(p, r, act) for p in nets], dim=1)
 
 
 def ae_forward(enc: Sequence[torch.Tensor], dec: Sequence[torch.Tensor], r: torch.Tensor) -> torch.Tensor:
@@ -172,16 +172,17 @@ class Preprocess(torch.nn.Module):
 # losses
 # --------------------------------------------------------------------------------------
 def eigen_loss(X, weight, nets, pp, alpha, eig_w, diag_coeff=None, beta=1.0, sort=True,
-               X_lagged=None, weight_lagged=None, lag_time=None):
+               X_lagged=None, weight_lagged=None, lag_time=None, act=torch.tanh):
     """EigenFunctionTask.loss_func (core.py:387-457).
 
     Returns (loss, eig_vals[k] sorted if ``sort``, non_penalty_loss, penalty, cvec).
     Generator branch when X_lagged is None (X must require grad), transfer-operator branch
     otherwise (lag_time = traj_dt * lag_idx).  The transfer-operator objective keeps the
-    reference's indexing (numerator idx, denominator cvec[idx], core.py:440).
+    reference's indexing (numerator idx, denominator cvec[idx], core.py:440).  ``act`` is the
+    activation between the layers of every network (the reference's ``activation`` argument).
     """
     k = len(nets)
-    y = eigen_forward(nets, pp(X))                                     # core.py:403
+    y = eigen_forward(nets, pp(X), act)                                # core.py:403
     tot_w = weight.sum()                                               # core.py:406
     mean = [(y[:, i] * weight).sum() / tot_w for i in range(k)]        # core.py:409
     var = [(y[:, i] ** 2 * weight).sum() / tot_w - mean[i] ** 2 for i in range(k)]  # core.py:410
@@ -195,7 +196,7 @@ def eigen_loss(X, weight, nets, pp, alpha, eig_w, diag_coeff=None, beta=1.0, sor
         eig = torch.tensor([float(dirich[i] / (tot_w * beta) / var[i]) for i in range(k)], dtype=X.dtype)  # :426
     else:
         tot_wl = weight_lagged.sum()
-        yl = eigen_forward(nets, pp(X_lagged))                         # core.py:414
+        yl = eigen_forward(nets, pp(X_lagged), act)                    # core.py:414
         mean_l = [(yl[:, i] * weight_lagged).sum() / tot_wl for i in range(k)]
         var_l = [(yl[:, i] ** 2 * weight_lagged).sum() / tot_wl - mean_l[i] ** 2 for i in range(k)]
         diff = [(((yl[:, i] - y[:, i]) ** 2) * weight).sum() for i in range(k)]

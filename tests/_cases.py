@@ -2,6 +2,9 @@
 import os
 
 import numpy as np
+import torch
+
+from oracle import ref_torch
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -77,7 +80,6 @@ def repeated_batch(D, B, seed, offset=0, device=None):
     """(X, w, w_agg, idx): X = D[idx] on the device with idx uniform over the M frames of D, random fp32 weights w, and the
     fp64 weight each distinct frame carries in total (host).  offset=1 returns a contiguous view that starts one frame into
     its allocation (not 16-byte aligned for 12 N-byte frames with N = 2 mod 4)."""
-    import torch
     device = torch.device("cuda", 0) if device is None else device
     D = torch.as_tensor(D, device=device)
     g = torch.Generator(device=device).manual_seed(seed)
@@ -94,3 +96,28 @@ def repeated_batch(D, B, seed, offset=0, device=None):
 def tol(gold, ref32, rel=1e-5, slack=1.0):
     """SURVEY 7.3-D: pass when |ours-gold| <= max(rel*|gold|, slack*|ref32-gold|)."""
     return max(rel * abs(float(gold)), slack * abs(float(ref32) - float(gold)))
+
+
+class GatheredFeatures(torch.nn.Module):
+    """Pre-processing of the gathered transfer-operator oracle: maps frame numbers (carried as float64, the dtype the
+    reference formula computes in) to precomputed fp64 features of the distinct frames."""
+
+    def __init__(self, R):
+        super().__init__()
+        self.R = torch.as_tensor(R, dtype=torch.float64)
+
+    def forward(self, i):
+        return self.R[i.long()]
+
+
+def lag_oracle(R, idx, w, nets, alpha, eig_w, lag, lag_time):
+    """fp64 transfer-operator loss of the batch X = D[idx] (frame t paired with t + lag) from the features R of the distinct
+    frames: reference formula (oracle/ref_torch.eigen_loss) on the gathered features.  Returns (comb-like dict, grads)."""
+    I = torch.as_tensor(np.asarray(idx), dtype=torch.float64)
+    wt = torch.as_tensor(np.asarray(w), dtype=torch.float64)
+    tn = [[torch.tensor(p, dtype=torch.float64, requires_grad=True) for p in n] for n in nets]
+    ref = ref_torch.eigen_loss(I[:-lag], wt[:-lag], tn, GatheredFeatures(R), alpha, eig_w, X_lagged=I[lag:],
+                               weight_lagged=wt[lag:], lag_time=lag_time)
+    ref[0].backward()
+    grads = [[np.zeros(tuple(t.shape)) if t.grad is None else t.grad.numpy() for t in n] for n in tn]
+    return dict(loss=float(ref[0]), eig=ref[1].numpy().astype(np.float64), cvec=[int(v) for v in ref[4]]), grads

@@ -8,7 +8,6 @@ import torch
 from oracle import closed_form as cf
 from oracle import ref_torch
 from tests import _cases as C
-from tests.test_step_at_scale_gpu import lag_oracle
 
 BASE = ref_torch.DIPEPTIDE_NM * 10.0
 
@@ -73,7 +72,7 @@ def test_gathered_lag_oracle_equals_reference_on_explicit_batch():
     pp = ref_torch.Preprocess(ref_torch.Align(BASE, list(range(22))), None)
     with torch.no_grad():
         R = pp(torch.as_tensor(D)).numpy()
-    gold, g_gold = lag_oracle(R, idx, w, nets, 20.0, [1.0, 0.6, 0.3], lag, tau)
+    gold, g_gold = C.lag_oracle(R, idx, w, nets, 20.0, [1.0, 0.6, 0.3], lag, tau)
     X, wt = torch.as_tensor(D[idx]), torch.as_tensor(w)
     tn = [[torch.tensor(p, dtype=torch.float64, requires_grad=True) for p in n] for n in nets]
     ref = ref_torch.eigen_loss(X[:-lag], wt[:-lag], tn, pp, 20.0, [1.0, 0.6, 0.3], X_lagged=X[lag:], weight_lagged=wt[lag:],

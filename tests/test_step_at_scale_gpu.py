@@ -131,31 +131,6 @@ def assert_bit_identical(a, b, tag):
             assert torch.equal(ta, tb), (tag, "gradients differ between runs")
 
 
-class GatheredFeatures(torch.nn.Module):
-    """Pre-processing of the gathered transfer-operator oracle: maps frame numbers (carried as float64, the dtype the
-    reference formula computes in) to precomputed fp64 features of the distinct frames."""
-
-    def __init__(self, R):
-        super().__init__()
-        self.R = torch.as_tensor(R, dtype=torch.float64)
-
-    def forward(self, i):
-        return self.R[i.long()]
-
-
-def lag_oracle(R, idx, w, nets, alpha, eig_w, lag, lag_time):
-    """fp64 transfer-operator loss of the batch X = D[idx] (frame t paired with t + lag) from the features R of the distinct
-    frames: reference formula (oracle/ref_torch.eigen_loss) on the gathered features.  Returns (comb-like dict, grads)."""
-    I = torch.as_tensor(np.asarray(idx), dtype=torch.float64)
-    wt = torch.as_tensor(np.asarray(w), dtype=torch.float64)
-    tn = [[torch.tensor(p, dtype=torch.float64, requires_grad=True) for p in n] for n in nets]
-    ref = ref_torch.eigen_loss(I[:-lag], wt[:-lag], tn, GatheredFeatures(R), alpha, eig_w, X_lagged=I[lag:],
-                               weight_lagged=wt[lag:], lag_time=lag_time)
-    ref[0].backward()
-    grads = [[np.zeros(tuple(t.shape)) if t.grad is None else t.grad.numpy() for t in n] for n in tn]
-    return dict(loss=float(ref[0]), eig=ref[1].numpy().astype(np.float64), cvec=[int(v) for v in ref[4]]), grads
-
-
 # --------------------------------------------------------------------------------------------- pre-processing of the cases
 def _chain(n):
     return bd.chain_structure(n, seed=100 + n)
@@ -381,5 +356,5 @@ def test_lag_loss_whole_tile_matches_gathered_oracle(case, tmp_path):
     idx, w = idx.cpu().numpy(), w.cpu().numpy().astype(np.float64)
     del X
     R = ppo.prepare(D_host.astype(np.float64))["r"]
-    gold, g64 = lag_oracle(R, idx, w, nets, 20.0, EIG_W[:k], lag, lag * dt)
+    gold, g64 = C.lag_oracle(R, idx, w, nets, 20.0, EIG_W[:k], lag, lag * dt)
     assert_eigen_envelope(out, grads, gold, g64, f"lag {case} B=2^17")
